@@ -349,9 +349,9 @@ def measure(E, workload, steps, warmup, local, dist=None, world=1, flags=0, e2e=
     dec_ms = barrier_max(dist, local, dec_ms)
     wall = barrier_max(dist, local, wall)
     value = aggregate_tokens_per_s(world, steps, n_dec, dec_ms)
-    res = {"value": value, "ms_per_step": wall * 1e3 / steps, "gpu_launches": int(launches), "launches_per_token": eng.launches_per_token,
-           "engine": eng.path, "path_calibration": eng.calibration, "dec_ms": dec_ms}
     timed_ids = ids.copy()
+    res = {"value": value, "ms_per_step": wall * 1e3 / steps, "gpu_launches": int(launches), "launches_per_token": eng.launches_per_token,
+           "engine": eng.path, "path_calibration": eng.calibration, "dec_ms": dec_ms, "ids": timed_ids[:seq]}
 
     if e2e:
         e2e_steps = max(1, min(steps, 2))
@@ -482,7 +482,7 @@ def tp_block(E, rank, world, local, dist):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps (each one full prompt + greedy decode run)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--workload", default="nano-168m-q80", choices=sorted(WORKLOADS))
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
@@ -495,7 +495,14 @@ def main():
     ap.add_argument("--no-pdl", action="store_true")
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--no-stream", action="store_true", help="forbid the streaming kernel")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed path returned in its last step (the token ids of the greedy decode) as DIR/ids.npy, "
+                         "float64; the inputs are seeded, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.mode != "replicas"):
+        ap.error("--dump-outputs writes the outputs of the default path (--impl b200 --mode replicas) only")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     preset, quant, gs, seq = WORKLOADS[args.workload]
@@ -527,6 +534,9 @@ def main():
         sampler.start()
     res = measure(E, args.workload, args.steps, args.warmup, local, dist, world, flags, parity=(rank == 0))
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "ids.npy"), res["ids"].astype(np.float64))
 
     tp = None
     if world > 1 and not args.no_extra:

@@ -6,9 +6,8 @@
  * reference's OWN headers and only LINKED against our library, so what must match is the ABI: struct layouts
  * (callers read ctx->llm->config.*, llm->arch/quant_type/group_size, ctx->tokenizer->vocab[], write
  * ctx->sampler->temperature/top_p and ctx->observation*: SURVEY finding 8) and the exported prototypes
- * (infer.h:253-282).  tests/test_boundary.py checks every size/offset below against the reference's
- * headers (through oracle/ref_harness.c:orh_abi_layout) whenever /root/reference is available, and against
- * the committed tests/golden/abi_layout.json otherwise.
+ * (infer.h:253-282).  tests/test_boundary.py checks every size/offset below against tests/golden/abi_layout.json,
+ * the layout read from the reference's own headers (oracle/ref_harness.c:orh_abi_layout).
  *
  * Private areas: nobody outside the reference's infer.c touches LLM.state (FwdBuffer) or LLM.params
  * (grep-verified in SURVEY finding 8); the shim keeps its engine handle and host logits buffer there.

@@ -2,10 +2,6 @@
 
     nano_b200/lib/libnano_b200.so        engine + C-ABI (include/nano_b200.h)        <- csrc/engine.cu, kernels.cuh
     nano_b200/lib/libnano_infer_b200.so  reference host API (infer.h symbols)        <- csrc/infer_b200.c
-    nano_b200/lib/libnano_refhost.so     the REFERENCE's own host objects that stay in the link line
-                                         (tokenizer.c utils.c hal_{ram,fs,os,misc}_linux.c), compiled unmodified
-                                         where they lie under /root/reference -- only when that tree exists
-    nano_b200/lib/nano_cli               infer/main_cli.c linked against our libraries ("nano_cli links unchanged")
 
 The outputs are git-ignored but travel to the GPU box with the gpurun snapshot.
 """
@@ -19,13 +15,9 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CSRC = os.path.join(ROOT, "nano_b200", "csrc")
 LIB = os.path.join(ROOT, "nano_b200", "lib")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
-REF = os.environ.get("NANO_REFERENCE", "/root/reference/infer")
 
 ENGINE_SO = os.path.join(LIB, "libnano_b200.so")
 SHIM_SO = os.path.join(LIB, "libnano_infer_b200.so")
-REFHOST_SO = os.path.join(LIB, "libnano_refhost.so")
-NANO_CLI = os.path.join(LIB, "nano_cli")
-REFHOST_SRCS = ["tokenizer.c", "utils.c", "hal_ram_linux.c", "hal_fs_linux.c", "hal_os_linux.c", "hal_misc_linux.c"]
 
 
 def _newer(target: str, sources) -> bool:
@@ -88,40 +80,11 @@ def build_shim(force: bool = False) -> str:
     return SHIM_SO
 
 
-def reference_present() -> bool:
-    return os.path.exists(os.path.join(REF, "main_cli.c"))
-
-
-def build_refhost(force: bool = False):
-    """The reference's unchanged host-side objects as a shared library (so ctypes can load the shim on the GPU box)."""
-    if not reference_present():
-        return REFHOST_SO if os.path.exists(REFHOST_SO) else None
-    srcs = [os.path.join(REF, s) for s in REFHOST_SRCS]
-    if force or _newer(REFHOST_SO, srcs):
-        subprocess.run(["gcc", "-DNANO_CLI", "-O2", "-w", "-fPIC", "-shared", "-pthread", "-I" + REF] + srcs +
-                       ["-o", REFHOST_SO, "-lm"], check=True)
-    return REFHOST_SO
-
-
-def build_nano_cli(force: bool = False):
-    """infer/Makefile:145-147 with `tensor.c infer.c` replaced by our two libraries."""
-    if not reference_present():
-        return NANO_CLI if os.path.exists(NANO_CLI) else None
-    srcs = [os.path.join(REF, s) for s in ["main_cli.c"] + REFHOST_SRCS]
-    if force or _newer(NANO_CLI, srcs + [SHIM_SO, ENGINE_SO]):
-        subprocess.run(["gcc", "-DNANO_CLI", "-O3", "-march=native", "-ffast-math", "-w", "-fopenmp", "-pthread", "-I" + REF] + srcs +
-                       ["-o", NANO_CLI, "-L" + LIB, "-lnano_infer_b200", "-lnano_b200", "-Wl,-rpath,$ORIGIN", "-lm"], check=True)
-    return NANO_CLI
-
-
 def build_all(force: bool = False, verbose: bool = False) -> None:
     build_engine(force, verbose)
     build_shim(force)
-    build_refhost(force)
-    build_nano_cli(force)
 
 
 if __name__ == "__main__":
     build_all(force="--force" in sys.argv, verbose="-v" in sys.argv)
-    print("built:", ENGINE_SO, SHIM_SO, REFHOST_SO if os.path.exists(REFHOST_SO) else "(no refhost)",
-          NANO_CLI if os.path.exists(NANO_CLI) else "(no nano_cli)")
+    print("built:", ENGINE_SO, SHIM_SO)

@@ -22,6 +22,8 @@ os.environ.setdefault("OMP_WAIT_POLICY", "passive")
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 REF_DIR = os.path.join(HERE, "_ref")
+NANO_CLI = os.path.join(HERE, "nano_cli")                   # the reference's main_cli.c linked against our libraries
+NANO_CLI_HOST = os.path.join(REF_DIR, "libnano_cli_host.a")  # its unmodified objects
 REFERENCE_SRC = "/root/reference/infer"
 
 f32p = C.POINTER(C.c_float)
@@ -38,6 +40,14 @@ def build(quiet: bool = True) -> None:
     """Compile the restatement and (when /root/reference exists) the reference flavours."""
     subprocess.run(["make", "-C", HERE, "-j4", "all"], check=True,
                    stdout=subprocess.DEVNULL if quiet else None)
+
+
+def link_nano_cli() -> str:
+    """Link oracle/nano_cli afresh from the reference's objects and our libraries (oracle/Makefile, target cli)."""
+    if os.path.exists(NANO_CLI):
+        os.remove(NANO_CLI)
+    subprocess.run(["make", "-C", HERE, "cli"], check=True, stdout=subprocess.DEVNULL)
+    return NANO_CLI
 
 
 def _ptr(a: np.ndarray, typ):

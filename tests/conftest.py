@@ -32,6 +32,31 @@ def sort_model():
     return open(os.path.join(GOLDEN, "sort6_model.bin"), "rb").read()
 
 
+_host_stub = None
+
+
+def load_host_stub():
+    """Compile tests/host_stub.c (allocation, sampler RNG, tokenizer: what a host program links beside the shim) in a
+    temporary directory and load it with RTLD_GLOBAL, so that libnano_infer_b200.so can be loaded and called.  The
+    directory is removed once the library is mapped."""
+    global _host_stub
+    if _host_stub is None:
+        import ctypes as C
+        import subprocess
+        import tempfile
+        with tempfile.TemporaryDirectory(prefix="nb200_host_stub_") as td:
+            so = os.path.join(td, "libnano_host_stub.so")
+            subprocess.run(["gcc", "-O2", "-Wall", "-fPIC", "-shared", "-I" + os.path.join(ROOT, "include"),
+                            os.path.join(ROOT, "tests", "host_stub.c"), "-o", so], check=True)
+            _host_stub = C.CDLL(so, mode=C.RTLD_GLOBAL)
+    return _host_stub
+
+
+def sha256(a) -> str:
+    import hashlib
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
 def bits(a):
     return np.ascontiguousarray(a, dtype=np.float32).view(np.uint32)
 

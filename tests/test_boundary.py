@@ -1,13 +1,11 @@
 """CPU tests for the drop-in boundary: ABI layout of include/nano_infer_abi.h == the reference's headers,
 libnano_infer_b200.so exports the reference API, and the reference's main_cli.c links against it unchanged."""
-import ctypes as C
 import json
 import os
 import re
 import subprocess
 import tempfile
 
-import numpy as np
 import pytest
 
 from conftest import GOLDEN, ROOT
@@ -23,17 +21,10 @@ def my_layout():
 
 
 def test_abi_layout_matches_committed_reference_layout():
+    """abi_layout.json: the sizes and offsets read from the reference's own headers (oracle/ref_harness.c:orh_abi_layout)."""
     want = json.load(open(os.path.join(GOLDEN, "abi_layout.json")))
+    assert len(want) > 60
     assert my_layout() == want
-
-
-@pytest.mark.skipif(not ob.ref_available("strict"), reason="oracle/_ref not built")
-def test_abi_layout_matches_reference_headers_live():
-    L = ob.RefEngine.lib("strict")
-    buf = (C.c_uint32 * 128)()
-    n = L.orh_abi_layout(buf, 128)
-    assert n > 60
-    assert my_layout() == list(buf)[:n]
 
 
 def exported_api():
@@ -62,9 +53,9 @@ def test_shim_exports_reference_api():
     assert "nb200_engine_create" in und and "oracle" not in subprocess.run(["ldd", nb_build.SHIM_SO], capture_output=True, text=True).stdout
 
 
-@pytest.mark.skipif(not nb_build.reference_present(), reason="/root/reference not present on this box")
+@pytest.mark.skipif(not os.path.exists(ob.NANO_CLI_HOST), reason="needs the reference's main_cli.c objects (oracle/Makefile)")
 def test_reference_nano_cli_links_unchanged():
-    exe = nb_build.build_nano_cli(force=True)
+    exe = ob.link_nano_cli()
     und = subprocess.run(["nm", "-D", "--undefined-only", exe], capture_output=True, text=True, check=True).stdout
     assert " U llm_context_init" in und and " U generate_sync" in und
     ldd = subprocess.run(["ldd", exe], capture_output=True, text=True).stdout
